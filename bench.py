@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — headline benchmark of the wavefront path tracer (contract: see the task statement / DESIGN.md §Measurement).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 Workload (config.workload): BASELINE.json configs[2] — the synthetic 1 387 526-triangle instanced scene, Disney BSDF + NEE,
@@ -21,6 +21,9 @@ roofline: the closest-hit traversal kernel: algorithmic bytes (SURVEY.md §8d: 4
 cpu_baseline: the CPU oracle (a port of the reference estimator; the reference's own `cpu` backend cannot be built here)
          on all host cores, on a bounded tile sample of the same frame.
 --impl reference: times that CPU implementation as its own arm (rank 0 only).
+--dump-outputs DIR: after the timed steps, rank 0 writes what a caller of the timed path receives - the normalised film
+         ([H, W, 4] float32, the sum over ranks for N > 1) - as DIR/film.npy.  The scene, seed and sample indices depend on
+         the arguments only, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -64,6 +67,13 @@ def workload_config(n_gpus: int) -> dict:
                      "than the 126 MB L2; no explicit flush",
         "host_buffers": "e2e: the host library's scene arrays and a reused film buffer, page-locked once by lrk (option pin_host_buffers)",
     }
+
+
+def dump_outputs(directory: str, film: np.ndarray) -> None:
+    """--dump-outputs: the film as DIR/film.npy ([HEIGHT, WIDTH, 4] float32, 33 MB)."""
+    out = Path(directory)
+    out.mkdir(parents=True, exist_ok=True)
+    np.save(out / "film.npy", np.ascontiguousarray(film, dtype=np.float32))
 
 
 class ClockSampler:
@@ -377,6 +387,8 @@ def run_ours(args, rank: int, world: int, local_rank: int):
     barrier()
     dt = time.perf_counter() - t0
     clock_info = clocks.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, r.film())
     st = r.stats()
     reduce_ms = st["reduce_ms"]
     r.set_option("time_kernels", 0)
@@ -559,7 +571,13 @@ def main():
     ap.add_argument("--impl", choices=["ours", "reference"], default="ours")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-configs", action="store_true", help="skip the short steps of the other BASELINE.json configurations")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the film of the timed steps as DIR/film.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        # that arm sizes its share of the frame by a timed calibration run, so its output is not the same from run to run
+        ap.error("--dump-outputs applies to --impl ours")
     from luisarender_b200 import distributed as D
 
     rank, world, local_rank = D.env_world()

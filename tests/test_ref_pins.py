@@ -94,7 +94,7 @@ def test_host_alias_table_matches_reference(golden):
     np.testing.assert_array_equal(pdf.view(np.uint32), golden["create_alias_table/pdf"].view(np.uint32))
 
 
-@pytest.mark.skipif(not G.LIB.exists(), reason="oracle/_ref/librefpins.so not built (needs /root/reference)")
+@pytest.mark.skipif(not G.LIB.exists(), reason="oracle/_ref/librefpins.so not built (needs a LuisaRender source tree: oracle/ref/README.md)")
 def test_fixture_is_what_the_reference_computes_now(golden):
     ref = G.RefPins()
     prob, alias, pdf = ref.create_alias_table(golden["create_alias_table/values"])

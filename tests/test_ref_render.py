@@ -90,7 +90,7 @@ def test_scene_text_in_the_fixture_is_the_generated_one(golden):
         assert bytes(golden[f"{name}/scene"]).decode() == source, name
 
 
-@pytest.mark.skipif(not G.CLI.exists(), reason="oracle/_ref/bin/luisa-render-cli not built (needs /root/reference)")
+@pytest.mark.skipif(not G.CLI.exists(), reason="oracle/_ref/bin/luisa-render-cli not built (needs a LuisaRender source tree: oracle/ref/README.md)")
 def test_fixture_is_what_the_reference_renders_now(golden):
     with tempfile.TemporaryDirectory() as tmp:
         for name in ("cornell_wavepath", "spheres_medium"):
